@@ -8,6 +8,7 @@ weights.  A "step" is one encoder-half forward (salience_transformer.py:106-183 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's sm_100a path
   python bench.py --impl reference ...                           # the reference's CPU path (oracle port), rank 0 only
   torchrun --nproc-per-node N bench.py --gpus N ...              # one process per GPU, weak scaling (replicas)
+  python bench.py ... --dump-outputs DIR                         # also write the last timed step's memory to DIR/memory.npy
 
 Prints ONE JSON line (rank 0).  value = device-resident throughput (CUDA-graph replay, inputs in HBM); e2e =
 same metric through EncoderRunner.run_host with pinned HOST buffers (H2D + forward + D2H inside the timed region);
@@ -545,6 +546,23 @@ def run_train(args, rank, world, local):
         dist.destroy_process_group()
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, outputs):
+    """Write each output the caller of the timed path receives as <out_dir>/<name>.npy in float32, so that two builds can be
+    compared output for output on the same seeded inputs.  The encoder memory of the benchmark's workload (2 x 22323 x 256)
+    is 45.7 MB and is written whole."""
+    import numpy as np
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -560,7 +578,11 @@ def main():
     ap.add_argument("--e2e-persistent-ctas", type=int, default=0,
                     help="cap of the persistent GEMM / FFN kernels during the e2e (multi-lane) measurement; 0 = one CTA per SM")
     ap.add_argument("--pipeline-depth", type=int, default=4, help="lanes of the host-buffer pipeline (e2e)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last timed step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     _claim_stdout()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -635,6 +657,8 @@ def main():
         clk.wait_first()
         total_ms = timed(runner.step, args.steps, args.warmup, on_start=clk.mark)
         clk.mark_end()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"memory": runner.memory})
         t_probe = time.time()
         while clk.proc is not None and clk.since_mark() < 3 and time.time() - t_probe < 3.0:  # same step, same flush, untimed
             with torch.cuda.stream(stream):
@@ -648,10 +672,10 @@ def main():
     # end to end through the public host-buffer API (the detector-side boundary, salience_detr.py:172-203: feature maps and
     # padding masks in, memory out; the sine position embedding is a function of the masks and is derived on the device).
     # Every step copies its feature maps from pinned host memory and its result back.  serial = one stream; pipelined =
-    # HostPipeline, double-buffered, copies overlap compute.  e2e is timed over >= 200 steps (round 1: 20 steps = 60 ms
-    # was too short to be stable across boxes).
+    # HostPipeline, double-buffered, copies overlap compute.  Every timed leg runs --steps steps; 20 steps (60 ms) proved
+    # too short for a stable e2e figure, so use >= 200 when e2e matters.
     from salience_detr_b200.runner import HostPipeline
-    e2e_steps = max(args.steps, 200)
+    e2e_steps = args.steps
     host_runner = EncoderRunner(model, feats, masks, None, use_graph=not args.no_graph, use_order=not args.no_order)
     host_runner.bind_host(feats_h)
     stream_keep, stream = stream, host_runner.stream
@@ -688,8 +712,8 @@ def main():
         out_pin.copy_(mem, non_blocking=True)
 
     stream_keep, stream = stream, torch.cuda.current_stream(dev)
-    fresh_ms = timed(fresh_step, max(10, args.steps // 2), 3)
-    fresh_serial_val = sdist.aggregate_throughput(bsz, max(10, args.steps // 2), world, fresh_ms)
+    fresh_ms = timed(fresh_step, args.steps, 3)
+    fresh_serial_val = sdist.aggregate_throughput(bsz, args.steps, world, fresh_ms)
     stream = stream_keep
     # the same, pipelined: copies, plan (own stream) and eager forwards of consecutive batches overlap; every batch still pays
     # its own plan and an eager forward
@@ -698,7 +722,7 @@ def main():
     fresh_batch = (feats_pin, masks_pin)
     fpipe.run([fresh_batch] * 6)
     barrier()
-    fresh_steps = max(args.steps, 100)
+    fresh_steps = args.steps
     t0 = torch.cuda.Event(enable_timing=True)
     t1 = torch.cuda.Event(enable_timing=True)
     t0.record()

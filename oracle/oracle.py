@@ -218,6 +218,8 @@ def msda_module(sd, pre, query, ref, value, shapes, lsi, mask, heads, levels, po
     loc = ref[:, :, None, :, None, :] + off / norm[None, None, None, :, None, :]
     if core == "torch":
         out = msda_core_torch(v, shapes.tolist(), loc, w)
+    elif callable(core):  # an operator with the `_C.ms_deform_attn_forward` contract (value, shapes, lsi, loc, attn)
+        out = core(v, shapes, lsi, loc, w)
     else:
         out = c_msda_forward(v, shapes, lsi, loc, w)
     return _lin(sd, pre + "output_proj", out)
@@ -481,3 +483,46 @@ def deterministic_state_dict(shapes: Dict[str, Sequence[int]], seed: int) -> Dic
             x = x / (shp[-1] ** 0.5)
         out[name] = x
     return out
+
+
+def golden_state_dict(shapes_json: str, seed: int, aliases_json: str = "{}") -> Dict[str, torch.Tensor]:
+    """The weights a golden fixture was made with: ``deterministic_state_dict`` of its stored shapes, with every key that is
+    the same tensor as another one in the reference model (e.g. ``encoder.enhance_mcsp`` = ``encoder_class_head``, reference
+    salience_transformer.py:79) set to the value that tensor ended up holding."""
+    import json
+    sd = deterministic_state_dict(json.loads(shapes_json), seed)
+    for k, src in json.loads(aliases_json).items():
+        sd[k] = sd[src]
+    return sd
+
+
+def sample_index(numel: int, n: int, seed: int) -> torch.Tensor:
+    """Fixed, seeded positions at which a golden fixture stores a large output (flat indices, at most ``n``)."""
+    return torch.randperm(numel, generator=torch.Generator().manual_seed(seed))[:n]
+
+
+def sampled(t: torch.Tensor, n: int, seed: int) -> torch.Tensor:
+    """``t`` (any device) at ``sample_index`` positions, on the CPU."""
+    return t.detach().reshape(-1)[sample_index(t.numel(), n, seed).to(t.device)].cpu()
+
+
+class TopDownNeck(torch.nn.Module):
+    """A small stand-in for the detector's neck (any module taking and returning ``{level: (b, C, h, w)}``, reference
+    salience_transformer.py:185-192): per level a channel mix, plus the nearest-upsampled result of the next coarser level,
+    then SiLU.  Weights come from ``seed``; channel mixes are matrix products, so they run in fp32 on any device."""
+
+    def __init__(self, channels: int, levels: int, seed: int = 3):
+        super().__init__()
+        g = torch.Generator().manual_seed(seed)
+        self.weight = torch.nn.Parameter(torch.randn(levels, channels, channels, generator=g) / channels ** 0.5)
+        self.bias = torch.nn.Parameter(0.1 * torch.randn(levels, channels, generator=g))
+
+    def forward(self, feats):
+        out, up = {}, None
+        for i in sorted(feats, reverse=True):
+            x = torch.einsum("oc,bchw->bohw", self.weight[i], feats[i]) + self.bias[i][None, :, None, None]
+            if up is not None:
+                x = x + F.interpolate(up, size=x.shape[-2:], mode="nearest")
+            up = F.silu(x)
+            out[i] = up
+        return {i: out[i] for i in sorted(out)}

@@ -18,10 +18,6 @@ import warnings
 
 _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASELINE_REF = os.path.join(_REPO, "baseline", "_ref")  # git-ignored install of the reference's hot-path modules
-# the Python modules of the path (SURVEY.md 8(c)); everything else of the reference stays where it is
-PATH_MODULES = ("base_transformer.py", "basic.py", "ms_deform_attn.py", "position_encoding.py", "salience_transformer.py")
-# consumer right after the path (SURVEY.md 8(f)-3): the RepVGG neck the encoder memory is handed to, for the hand-off test
-NECK_MODULES = (("models/necks", "repnet.py"), ("models/bricks", "misc.py"))
 
 
 def _has(root: str) -> bool:
@@ -43,36 +39,6 @@ REFERENCE_ROOT = _resolve_root()
 
 def available() -> bool:
     return _has(REFERENCE_ROOT)
-
-
-def install(src: str = "/root/reference", dst: str = BASELINE_REF) -> bool:
-    """Install the UNMODIFIED Python modules of the path from the reference tree into the git-ignored
-    ``baseline/_ref`` (which travels to the GPU box; /root/reference does not).  The reference has no setup.py /
-    pyproject, so `pip install --target` does not apply: this copies the five files byte for byte.  The CUDA
-    extension sources (models/bricks/ops/cuda) are NOT installed: they do not compile against torch 2.11 (SURVEY.md
-    fact 2), so the reference's own `load(...)` fails, warns and falls back to its pure-PyTorch MSDA
-    (ms_deform_attn.py:13-26,361-372) -- which is the path the reference really runs on this image."""
-    import filecmp
-    import shutil
-
-    if not _has(src):
-        return _has(dst)
-    out = os.path.join(dst, "models", "bricks")
-    os.makedirs(out, exist_ok=True)
-    for name in PATH_MODULES:
-        a, b = os.path.join(src, "models", "bricks", name), os.path.join(out, name)
-        if not (os.path.exists(b) and filecmp.cmp(a, b, shallow=False)):
-            shutil.copyfile(a, b)
-    for sub, name in NECK_MODULES:
-        a, b = os.path.join(src, sub, name), os.path.join(dst, sub, name)
-        os.makedirs(os.path.dirname(b), exist_ok=True)
-        if os.path.exists(a) and not (os.path.exists(b) and filecmp.cmp(a, b, shallow=False)):
-            shutil.copyfile(a, b)
-    with open(os.path.join(dst, "README"), "w") as f:
-        f.write("Unmodified copies of xiuqhou/Salience-DETR models/bricks/{%s} (reference arm of bench.py and the\n"
-                "drop-in tests; written by oracle/ref_import.install(), git-ignored, never imported by the product).\n"
-                % ",".join(PATH_MODULES))
-    return True
 
 
 def _install_stub():

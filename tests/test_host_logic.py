@@ -184,3 +184,18 @@ def test_bench_stdout_carries_only_the_result_line():
     assert p.stdout.decode() == '{"ok": 1}\n'
     err = p.stderr.decode()
     assert "banner from a C library" in err and "a python print" in err
+
+
+def test_bench_dump_outputs(tmp_path):
+    """`bench.py --dump-outputs DIR`: every output as DIR/<name>.npy in float32, values unchanged; more than 64 MiB in all is
+    refused before anything is written."""
+    import numpy as np
+    import pytest
+    import bench
+    mem = torch.randn(2, 37, 8, dtype=torch.float64)
+    bench.dump_outputs(str(tmp_path / "out"), {"memory": mem})
+    got = np.load(tmp_path / "out" / "memory.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, mem.float().numpy())
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "big"), {"memory": torch.empty(bench.DUMP_LIMIT_BYTES // 4 + 1)})
+    assert not (tmp_path / "big").exists()
